@@ -14,6 +14,10 @@ one batch of `--pairs-per-step` synthetic pairs, through the C ABI (include/chro
           the reference's own per-batch "Mapped N read pairs in Xs" lines.
 
 Prints ONE JSON line on rank 0.
+
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the headline (device) leg computed in its last step -- every
+          field of the records and every count the call returns -- as DIR/<name>.npy in float64, so that two builds can be
+          compared output for output on identical seeded inputs (see dump_outputs()).
 """
 import argparse
 import json
@@ -415,6 +419,8 @@ def run_ours(a):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             dt = float(t.item())
         res[name] = dict(dt=dt, stage=stage, n_rec=n_rec, n_map=n_map, clocks=sampler.summary(), steps=steps)
+        if name == "device" and a.dump_outputs:  # the last timed step's records, before the next leg overwrites out_dev
+            last = (out_dev[:st["n_records"] * 24].cpu().numpy().view(rec_dtype), st)
     # ---- the one collective of the multi-GPU path (SURVEY.md 8e), outside the timed mapping region: duplicate removal over the
     # records of up to four mapped batches per rank: tuple pack -> ONE ncclAllGather -> radix sort + survivor rule on the GPU
     exchange = None
@@ -566,9 +572,30 @@ def run_ours(a):
         line["dedup_exchange"] = exchange
     if cpu_baseline:
         line["cpu_baseline"] = cpu_baseline
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, *last)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, recs, stats):
+    """One float64 .npy per record field and one per count of `stats`, all together under DUMP_BYTES: a larger output is reduced
+    to a sample of its records drawn with a fixed seed; sample_index.npy holds the sampled positions (all of them when nothing
+    was dropped)."""
+    os.makedirs(d, exist_ok=True)
+    n = len(recs)
+    cap = (DUMP_BYTES - (64 << 10)) // (8 * (len(recs.dtype.names) + 1))  # 64 KB left for the counts and the .npy headers
+    idx = np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+    np.save(os.path.join(d, "sample_index.npy"), idx.astype(np.float64))
+    for f in recs.dtype.names:
+        np.save(os.path.join(d, f + ".npy"), recs[f][idx].astype(np.float64))
+    for k, v in stats.items():
+        np.save(os.path.join(d, k + ".npy"), np.array([v], dtype=np.float64))
+    log("outputs of the last timed step (%d of %d records) written to %s" % (len(idx), n, d))
 
 
 def cpu_port_baseline(a, m, ref, offsets, seq_len, host_batch):
@@ -734,7 +761,10 @@ def main():
     ap.add_argument("--cells", type=int, default=10000)
     ap.add_argument("--workdir", default=None)
     ap.add_argument("--reference-index", default="ours", choices=["ours", "chromap"], help="--impl reference: who builds the index the reference binary loads")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's records and counts to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if a.warmup < 3:
         a.warmup = 3
     if a.impl == "reference":

@@ -77,3 +77,5 @@ $REF -q 0 --remove-pcr-duplicates --Tn5-shift -x ref.index -r ref.fa -1 read1.fq
 md5sum *.bed > md5.txt
 gzip -9 -n ref.fa read1.fq read2.fq barcode.fq *.bed
 rm -f ref.index
+# what `chromap -i` writes, as digests (the index files themselves are too large to store)
+python $REPO/tests/golden/make_index_digests.py

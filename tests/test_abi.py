@@ -93,20 +93,18 @@ def test_host_sam_writer_reproduces_reference_text(golden_dir, case, kw, paired)
     assert text == gzip.open(os.path.join(d, case + ".sam.gz")).read()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference headers (build container only)")
-def test_integration_stub_compiles_against_the_reference_headers(tmp_path):
-    """The bridge shown in INTEGRATION.md is real code: it type-checks against the reference's own headers."""
-    import subprocess
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    md = open(os.path.join(root, "INTEGRATION.md")).read()
-    a = md.index("```cpp") + 6
-    code = md[a:md.index("```", a)].replace('#include "chromap_b200.h"', "")
-    src = tmp_path / "bridge.cc"
-    src.write_text("#include <cstdint>\n#include <string>\n#include <vector>\n#include \"mapping_parameters.h\"\n#include \"sequence_batch.h\"\n"
-                   "#include \"bed_mapping.h\"\n#include \"utils.h\"\n#include \"chromap_b200.h\"\nnamespace chromap {\n" + code + "\n}\nint main() { return 0; }\n")
-    r = subprocess.run(["/usr/bin/g++", "-std=c++11", "-fsyntax-only", "-I/root/reference/src", "-I" + os.path.join(root, "include"), str(src)],
-                       capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[:2000]
+def test_integration_stub_compiles_against_the_reference_headers():
+    """The bridge shown in INTEGRATION.md is real code: it type-checks against the reference's own headers.  Those headers cannot
+    be stored here, so the check runs where build() compiles the reference binary (oracle/Makefile, target ref) and records its
+    result in oracle/_ref/integration_bridge.txt; this test holds the current INTEGRATION.md and include/chromap_b200.h to it."""
+    from oracle import integration_bridge
+    p = os.path.join(ROOT, "oracle", "_ref", "integration_bridge.txt")
+    if not os.path.exists(p):
+        pytest.skip("the reference's headers were absent when the project was built (oracle/Makefile, target ref)")
+    head, _, diagnostics = open(p).read().partition("\n")
+    checked, rc = head.split()
+    assert checked == integration_bridge.digest(), "INTEGRATION.md or include/chromap_b200.h changed since the check: run build() again"
+    assert rc == "0", diagnostics
 
 
 @pytest.mark.parametrize("kw,paired", [(dict(preset="", max_num_best_mappings=3, mapq_threshold=0), True), (dict(preset="atac"), True),

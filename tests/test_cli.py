@@ -8,7 +8,6 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CLI = os.path.join(ROOT, "chromap_b200", "bin", "chromap-b200")
-REF_BIN = os.path.join(ROOT, "oracle", "_ref", "chromap")
 
 
 def _ensure_cli():
@@ -57,20 +56,28 @@ def test_cli_end_to_end_equals_reference_binary_output(case, args, tmp_path, gol
 
 @pytest.mark.gpu
 def test_index_file_written_by_cli_is_loadable_by_the_reference_binary(tmp_path, golden_dir):
-    """Index::Load + kh_get of the unmodified reference must find every key in the file we write."""
-    if not os.path.exists(REF_BIN):
-        pytest.skip("oracle/_ref/chromap not built")
+    """The file we write is what the unmodified reference's `chromap -i` writes for the same FASTA, up to the bucket order inside
+    khash's arrays: the same header (k, w, kh_size, n_buckets, size, n_occupied, upper_bound), the same length, the same key ->
+    value map and occurrence table (synth_small/ref_index.json holds the reference's side, tests/golden/make_index_digests.py).
+    A reader of the format (the oracle's restatement of Index::Load) maps through it to the reference binary's BED."""
+    import json
+    import numpy as np
+    from oracle import oracle_py as orc
+    from tests.util import index_digest
     cli = _ensure_cli()
     d = os.path.join(golden_dir, "synth_small")
+    want = json.load(open(os.path.join(d, "ref_index.json")))
     ref = str(tmp_path / "ref.fa")
     open(ref, "wb").write(gzip.open(os.path.join(d, "ref.fa.gz")).read())
-    for n in ("read1", "read2"):
-        open(str(tmp_path / (n + ".fq")), "wb").write(gzip.open(os.path.join(d, n + ".fq.gz")).read())
     idx = str(tmp_path / "ref.index")
     subprocess.check_call([cli, "-i", "-r", ref, "-o", idx], stderr=subprocess.DEVNULL)
+    raw = open(idx, "rb").read()
+    assert len(raw) == want["file_bytes"]
+    assert [int(x) for x in np.frombuffer(raw[:8], "<i4")] + [int(x) for x in np.frombuffer(raw[8:28], "<u4")] == want["header"]
+    got = index_digest(orc.Index(idx).arrays())
+    assert got == {f: want[f] for f in got}
     out = str(tmp_path / "ref_out.bed")
-    subprocess.check_call([REF_BIN, "-x", idx, "-r", ref, "-1", str(tmp_path / "read1.fq"), "-2", str(tmp_path / "read2.fq"), "-o", out, "-t", "2"],
-                          stderr=subprocess.DEVNULL)
+    orc.run_files(orc.make_params(""), idx, ref, os.path.join(d, "read1.fq.gz"), os.path.join(d, "read2.fq.gz"), out, n_threads=2)
     assert open(out, "rb").read() == gzip.open(os.path.join(d, "default.bed.gz")).read()
 
 

@@ -232,55 +232,39 @@ def test_index_built_on_device_equals_reference_semantics(synth):
     assert bed == gzip.open(os.path.join(synth["d"], "default.bed.gz")).read()
 
 
-def test_device_built_index_has_the_content_of_the_reference_binarys_index(tmp_path):
-    """`chromap -i` (the unmodified reference binary, oracle/_ref) and cmx_build_index on the same 20 Mbp reference with planted
-    repeats and N runs: same k / w, same bucket count, the SAME occurrence table byte for byte, and every key of the reference's
-    hash table present on the device with the same value (and no other key).  Only the bucket ORDER inside khash's arrays is not
-    compared: it is a function of khash's resize history (kh_resize re-inserts in bucket order), not of the content; lookups do
-    not depend on it.  This is what lets bench.py's reference arm run on an index written by cmx_download_index."""
-    import subprocess
-    binp = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "chromap")
-    if not os.path.exists(binp):
-        pytest.skip("oracle/_ref/chromap not built")
-    rng = np.random.default_rng(3)
-    seqs = []
-    fam = rng.integers(0, 4, 300)
-    for si in range(4):
-        s = rng.integers(0, 4, 5000000)
-        seg = rng.integers(0, 4, 5000)
-        for st in rng.integers(0, len(s) - 5000, 30):
-            s[st:st + 5000] = seg
-        for st in rng.integers(0, len(s) - 300, 800):
-            s[st:st + 300] = fam
-        a = np.frombuffer(b"ACGT", dtype=np.uint8)[s].copy()
-        for st in rng.integers(0, len(a) - 200, 40):
-            a[st:st + int(rng.integers(1, 200))] = ord("N")
-        seqs.append(a)
+def test_device_built_index_has_the_content_of_the_reference_binarys_index(tmp_path, golden_dir):
+    """`chromap -i` (the unmodified reference binary) and cmx_build_index on the same 20 Mbp reference with planted repeats and
+    N runs: same k / w, same bucket count, the SAME occurrence table byte for byte, and the same key -> value map (no other key),
+    every key found by the device's probe with its value.  The reference binary's side is stored as digests plus a sample of its
+    (key, value) pairs (tests/golden/planted_20mbp_index.json, written by tests/golden/make_index_digests.py).  Only the bucket
+    ORDER inside khash's arrays is not compared: it is a function of khash's resize history (kh_resize re-inserts in bucket
+    order), not of the content; lookups do not depend on it.  This is what lets bench.py's reference arm run on an index
+    written by cmx_download_index."""
+    import hashlib
+    import json
+    from tests.util import index_digest, planted_repeat_reference, write_fasta
+    want = json.load(open(os.path.join(golden_dir, "planted_20mbp_index.json")))
+    names, seqs = planted_repeat_reference()
     fa = tmp_path / "ref.fa"
-    with open(fa, "wb") as f:
-        for i, a in enumerate(seqs):
-            f.write(b">s%d\n" % i); a.tofile(f); f.write(b"\n")
-    idx = tmp_path / "ref.index"
-    r = subprocess.run([binp, "-i", "-r", str(fa), "-o", str(idx)], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-500:]
-    a = orc.Index(str(idx)).arrays()
+    write_fasta(fa, names, seqs)
+    assert hashlib.sha256(fa.read_bytes()).hexdigest() == want["fasta_sha256"], "not the reference the digests were made from"
+    k_mer, window = want["header"][:2]
     m = cb.Mapper(cb.make_params("", max_read_length=64))
-    m.upload_reference(seqs, ["s%d" % i for i in range(len(seqs))])
-    m.build_index(17, 7)
+    m.upload_reference(seqs, names)
+    m.build_index(k_mer, window)
     info = m.index_info()
     d = m.download_index()
-    assert d["n_buckets"] == a["n_buckets"]
-    assert info["n_occ"] == len(a["occ"]) and np.array_equal(d["occ"], a["occ"])
-    nb = a["n_buckets"]
-    occupied = ((a["flags"][np.arange(nb) >> 4] >> ((np.arange(nb) & 15) << 1)) & 3) == 0
-    keys, vals = a["keys"][occupied], a["vals"][occupied]
-    assert len(keys) == info["n_keys"] == d["n_keys"]
+    got = index_digest(d)
+    assert got == {f: want[f] for f in got}
+    assert info["n_occ"] == want["n_occ"] and info["n_keys"] == d["n_keys"] == want["n_keys"]
+    sk, sv = np.array(want["sample_keys"], dtype=np.uint64), np.array(want["sample_vals"], dtype=np.uint64)
+    f, k, v = m.stage_probe(sk >> np.uint64(1))
+    assert f.all() and np.array_equal(k, sk) and np.array_equal(v, sv)
+    nb = d["n_buckets"]
+    occ_d = ((d["flags"][np.arange(nb) >> 4] >> ((np.arange(nb) & 15) << 1)) & 3) == 0
+    keys, vals = d["keys"][occ_d], d["vals"][occ_d]
     f, k, v = m.stage_probe(keys >> np.uint64(1))
     assert f.all() and np.array_equal(k, keys) and np.array_equal(v, vals)
-    # the file layout we write holds the same multiset of (key, value) pairs
-    occ_d = ((d["flags"][np.arange(nb) >> 4] >> ((np.arange(nb) & 15) << 1)) & 3) == 0
-    o1, o2 = np.argsort(keys), np.argsort(d["keys"][occ_d])
-    assert np.array_equal(keys[o1], d["keys"][occ_d][o2]) and np.array_equal(vals[o1], d["vals"][occ_d][o2])
 
 
 def test_reference_quickstart_golden(golden_dir):

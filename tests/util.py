@@ -59,3 +59,43 @@ def load_pairs(d, r1="read1.fq.gz", r2="read2.fq.gz"):
     s1, o1 = pack(a)
     s2, o2 = pack(b)
     return s1, o1, s2, o2
+
+
+def planted_repeat_reference():
+    """4 x 5 Mbp of random bases (seed 3) with planted 5 kb segmental repeats, a 300 bp family and N runs: (names, seqs)."""
+    rng = np.random.default_rng(3)
+    seqs = []
+    fam = rng.integers(0, 4, 300)
+    for si in range(4):
+        s = rng.integers(0, 4, 5000000)
+        seg = rng.integers(0, 4, 5000)
+        for st in rng.integers(0, len(s) - 5000, 30):
+            s[st:st + 5000] = seg
+        for st in rng.integers(0, len(s) - 300, 800):
+            s[st:st + 300] = fam
+        a = np.frombuffer(b"ACGT", dtype=np.uint8)[s].copy()
+        for st in rng.integers(0, len(a) - 200, 40):
+            a[st:st + int(rng.integers(1, 200))] = ord("N")
+        seqs.append(a)
+    return ["s%d" % i for i in range(len(seqs))], seqs
+
+
+def write_fasta(path, names, seqs):
+    with open(path, "wb") as f:
+        for n, a in zip(names, seqs):
+            f.write(b">%s\n" % n.encode()); a.tofile(f); f.write(b"\n")
+
+
+def index_digest(a):
+    """What an index (n_buckets / flags / keys / vals / occ arrays in khash's layout) holds, independent of the bucket order
+    inside khash's arrays (a function of its resize history, not of the content): the bucket count, the key -> value map and the
+    occurrence table, each as a sha256 with its size."""
+    import hashlib
+    nb = int(a["n_buckets"])
+    b = np.arange(nb)
+    occupied = ((a["flags"][b >> 4] >> ((b & 15) << 1)) & 3) == 0
+    keys, vals = a["keys"][occupied].astype("<u8"), a["vals"][occupied].astype("<u8")
+    o = np.argsort(keys)
+    return dict(n_buckets=nb, n_keys=int(len(keys)), n_occ=int(len(a["occ"])),
+                keys_vals_sha256=hashlib.sha256(keys[o].tobytes() + vals[o].tobytes()).hexdigest(),
+                occ_sha256=hashlib.sha256(np.ascontiguousarray(a["occ"], dtype="<u8").tobytes()).hexdigest())
